@@ -91,7 +91,12 @@ def parse():
                     "(collectives replaced by local copies); the line is marked emulated")
     ap.add_argument("--cpu-sample-targets", type=int, default=1_000_000)
     ap.add_argument("--cpu-sample-queries", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed paths computed in their last step to DIR/<name>.npy (float32/float64): the top-k scores "
+                         "and ids of the headline step and, if train steps ran, a fixed row sample of the parameters they updated")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     a.cfg = dict(CONFIGS[a.config])
     if a.targets:
         a.cfg["targets"] = a.targets
@@ -484,6 +489,11 @@ def run_b200(args):
     h.set_option("pad_skip", 0)                  # FULL regime: all T steps are executed, as the reference does
     l0 = total_launches()
     ms_dev, dev_samples = timed(step_device, args.steps, W, args.repeats)
+    dump = {}
+    if args.dump_outputs and rank == 0:          # the last timed step's result, before later regions reuse the buffers
+        src_s, src_i = (fs, fi) if G > 1 else (sc, ix)
+        dump["top_scores"] = src_s.cpu().numpy().astype(np.float32)
+        dump["top_ids"] = src_i.cpu().numpy().astype(np.float64)
     n_steps_run = sum([args.steps + (W if i == 0 else min(W, 1)) for i in range(max(1, args.repeats))])
     launches_per_step = (total_launches() - l0) / float(n_steps_run)
     ms_e2e, e2e_samples = timed(step_e2e, args.steps, W, args.repeats)
@@ -609,6 +619,21 @@ def run_b200(args):
                  "pair_rows_per_gpu": Bt, "pair_rows_global": Bt * world, "positives_per_gpu": n_pos, "dtype": "bf16 operands / f32 accumulate, state, stash and optimizer (tcgen05 GEMMs)" if Bt % 8 == 0 and WE % 8 == 0 and H % 8 == 0 else "f32",
                  "flops_per_step": fl, "achieved_tflops": fl / (ms_t / args.train_steps * 1e-3) / 1e12,
                  "parallelism": "data-parallel x%d, all-reduce of the gradient arena" % world if world > 1 else "single GPU"}
+        if args.dump_outputs and rank == 0:      # the parameters the last train step wrote; large tables as a fixed row sample
+            rng_d = np.random.default_rng(0)
+            for name, _ in h.param_names():
+                v = h.get_param(name)
+                if v.ndim and v.shape[0] > 4096:
+                    v = v[np.sort(rng_d.choice(v.shape[0], 4096, replace=False))]
+                dump["param." + name.replace("/", ".")] = v.astype(np.float32)
+
+    if dump:
+        total = sum(v.nbytes for v in dump.values())
+        if total > 64 << 20:
+            raise SystemExit("bench.py: --dump-outputs: %d bytes exceed 64 MB" % total)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, v in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), v)
 
     if rank != 0:
         if world > 1:
